@@ -22,6 +22,9 @@ re-schedule → unbind), like FairSchedulingAlgo.Schedule walks the pools of a c
 
 `--impl reference` times the oracle port on the same cycle (the same pools one after the other, the
 way the reference schedules them) on the host cores; rank 0 only.
+
+`--dump-outputs DIR` writes what the last timed device-resident cycle computed (see dump_outputs) so
+that two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -33,6 +36,9 @@ import subprocess
 import sys
 import threading
 import time
+
+# The tree may be read-only where the benchmark runs, and it must be left as build() left it.
+sys.dont_write_bytecode = True
 
 # Before anything creates the CUDA context: one hardware work queue per concurrent round (the pools
 # of a cycle run on one stream each; with the default of 8 queues two of them can share one).
@@ -264,6 +270,53 @@ def extra_workload(dev, name, parity_name=None, steps=2):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, pools, results, inputs, job_sample=1 << 16, node_sample=1 << 13):
+    """Write the output arrays a caller receives from armada_round_download for each pool in `pools`
+    (results[i] belongs to pools[i]) as DIR/<name>.npy in float64, with the pool as the leading axis.
+    Each pool's job and node axes are cut to a fixed sample (seed 0, sorted, the same in every run;
+    job_sample.npy / node_sample.npy hold the indices); the sample is halved until the whole dump
+    fits in DUMP_LIMIT_BYTES.  Integers are exact below 2**53; larger resource totals are rounded to
+    float64.  The scalar results go to num_*.npy / termination_reason.npy with shape (pools,)."""
+    from armada_b200.model import RoundResult
+    inp0 = inputs[pools[0]]
+    names = [n for n in RoundResult.ARRAYS if n != "job_excluded_nodes" or inp0.collect_excluded_nodes]
+    if results[0].first_pass:
+        names += ["job_seq_first_pass", "job_reason_first_pass"]
+    while True:
+        out = {"pool": np.asarray(pools, np.float64)}
+        kj = min([job_sample] + [int(inputs[p].num_jobs) for p in pools])
+        kn = min([node_sample] + [int(inputs[p].num_nodes) for p in pools])
+        jidx = [np.sort(np.random.default_rng(0).choice(int(inputs[p].num_jobs), kj, replace=False)) for p in pools]
+        nidx = [np.sort(np.random.default_rng(0).choice(int(inputs[p].num_nodes), kn, replace=False)) for p in pools]
+        out["job_sample"] = np.stack(jidx).astype(np.float64)
+        out["node_sample"] = np.stack(nidx).astype(np.float64)
+        for n in names:
+            rows = []
+            for res, ji, ni in zip(results, jidx, nidx):
+                a = getattr(res, n)
+                if n.startswith("job_"):
+                    a = a[ji]
+                elif n == "node_alloc":
+                    a = a[..., ni]
+                rows.append(a.astype(np.float64))
+            out[n] = np.stack(rows)
+        for n in RoundResult.SCALARS:
+            out[n] = np.asarray([getattr(res.out, n) for res in results], np.float64)
+        total = sum(a.nbytes for a in out.values())
+        if total <= DUMP_LIMIT_BYTES:
+            break
+        if job_sample <= 1 and node_sample <= 1:
+            raise SystemExit(f"--dump-outputs: {total} bytes even with one job and one node per pool")
+        job_sample, node_sample = max(1, job_sample // 2), max(1, node_sample // 2)
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in out.items():
+        np.save(os.path.join(out_dir, f"{n}.npy"), a)
+    return total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -274,7 +327,10 @@ def main():
     ap.add_argument("--pools", type=int, default=8, help="pools per scheduling cycle (fixed: strong scaling over GPUs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed cycle as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and at least one timed step")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -381,6 +437,9 @@ def main():
         e2e_placed += sum(int(out[p].stats.placements) for p in mine)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # the resident contexts still hold the last timed resident cycle (the end-to-end leg uses its own)
+        dump_outputs(args.dump_outputs, mine, [cyc.download_resident(i) for i in range(len(mine))], inputs)
 
     tm = torch.tensor([dev_ms, e2e_s * 1e3, pass_ms], dtype=torch.float64, device="cuda")
     cnt = torch.tensor([placements, e2e_placed, probes, launches], dtype=torch.float64, device="cuda")

@@ -1,10 +1,10 @@
 #!/usr/bin/env python3
 """Extract the reference's table-driven test vectors into JSON golden fixtures.
 
-Run in the BUILD container (where /root/reference is mounted); the JSON it writes is
-committed under tests/golden/ and is all that travels to the GPU box:
+Run it against a checkout of armadaproject/armada; the JSON it writes is committed under
+tests/golden/ and is all the tests read:
 
-    python tests/golden/extract_go_tables.py
+    python tests/golden/extract_go_tables.py <path to the armada checkout>
 
 The Go test files declare their known-answer tables as composite literals
 (`tests := map[string]struct{...}{ "name": {Field: expr, ...}, ... }`).  This script parses
@@ -28,7 +28,7 @@ import os
 import re
 import sys
 
-REF = "/root/reference/internal/scheduler"
+REF = os.path.join(sys.argv[1] if len(sys.argv) > 1 else ".", "internal", "scheduler")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 TABLES = [
